@@ -2,6 +2,7 @@
 """bench.py -- matched image-pairs / second on the compute-matches hot path (BASELINE.json metric).
 
     python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload c3|c2|c2-msurf64|c4|c4-exact] [--matcher exact|cascade]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (default): BASELINE.json configs[2] = **C3**, the configuration the north_star target is quoted on:
@@ -183,6 +184,42 @@ def first_pairs(m, n):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, pairs, parts, max_matches_per_pair):
+    """--dump-outputs: the PairWiseMatches of the last timed step, as float64 .npy files (indices are exact in float64).
+        pairs.npy          [P, 2]  the step's pair list (I, J)
+        match_counts.npy   [P]     matches of each pair (0 for a pair absent from the map)
+        sample_pairs.npy   [S]     rows of pairs.npy: a fixed, seeded sample of the pairs
+        sample_offsets.npy [S + 1] CSR offsets of the sampled pairs into sample_matches.npy
+        sample_matches.npy [M, 2]  (i, j) of every match of the sampled pairs, in the order the map holds them
+    parts: [(pairs, ofs, matches)] per rank in pair order (Matches.export_csr / sharding.Gather.result).  S depends on
+    the workload's shape alone (S pairs of max_matches_per_pair matches fit DUMP_BYTES), so two builds run on the same
+    arguments dump the same sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    pairs = np.asarray(pairs, np.int64).reshape(-1, 2)
+    mp = np.concatenate([p[0].reshape(-1, 2) for p in parts]).astype(np.int64)
+    cnt = np.concatenate([np.diff(p[1].astype(np.int64)) for p in parts])
+    mm = np.concatenate([p[2] for p in parts])
+    ofs = np.concatenate([[0], np.cumsum(cnt)])
+    row_of = {(I, J): r for r, (I, J) in enumerate(mp.tolist())}
+    row = np.array([row_of.get((I, J), -1) for I, J in pairs.tolist()], np.int64)    # -1: pair absent from the map
+    counts = np.append(cnt, 0)[row]
+    P = len(pairs)
+    fixed = 8 * (3 * P + 1)
+    S = int(min(P, max(0, DUMP_BYTES - fixed) // (16 * max_matches_per_pair + 16)))
+    sel = np.sort(np.random.default_rng(20260924).choice(P, S, replace=False))
+    chunks = [mm[ofs[row[k]]:ofs[row[k] + 1]] for k in sel if row[k] >= 0]
+    sm = np.concatenate(chunks) if chunks else np.zeros(0, mm.dtype)
+    out = {"pairs": pairs, "match_counts": counts, "sample_pairs": sel,
+           "sample_offsets": np.concatenate([[0], np.cumsum(counts[sel])]),
+           "sample_matches": np.stack([sm["i"], sm["j"]], 1)}
+    assert sum(a.size * 8 for a in out.values()) <= DUMP_BYTES
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def cpu_match_sample(po, sc, sample, n_threads):
     """The oracle port on `sample` pairs, one pair after another, upstream's own `#pragma omp parallel for` over the
     queries of SearchNeighbours using all n_threads (the outer omp-over-J team of src/R3DComputeMatches.cpp:465 would
@@ -248,7 +285,11 @@ def main():
                     help="exact = tensor-core brute force (default); cascade = OpenMVG CASCADE_HASHING_L2 (default of c4)")
     ap.add_argument("--feats", type=int, default=0, help="experiment only")
     ap.add_argument("--images", type=int, default=0, help="experiment only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the matches of the last timed step to DIR/<name>.npy (float64, <= 64 MB; see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; it does not apply to --impl reference")
     # stdout carries exactly ONE line (the JSON): anything a library prints there (NCCL's version banner
     # at communicator creation, ...) is sent to stderr instead
     real_stdout = os.dup(1)
@@ -355,6 +396,9 @@ def main():
     barrier()
     t_res = time.perf_counter() - t0
     n_matches, n_match_pairs = sum_over_ranks(m.total, m.num_pairs)
+    if args.dump_outputs and rank == 0:     # what rank 0 holds after the last step: the gathered map when N > 1
+        dump_outputs(args.dump_outputs, pairs, gather.result() if gather is not None else [m.export_csr()],
+                     int(counts.max()))
 
     # ---------------- end-to-end leg: `e2e` ----------------
     for _ in range(2):

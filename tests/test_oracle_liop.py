@@ -1,15 +1,18 @@
 """LIOP-144 descriptor stage (SURVEY.md 8f-1): the oracle's restatement against THE REFERENCE ITSELF.
 
 `r3d_vl_liopdesc_process` is the one piece of reference arithmetic on the path that compiles standalone
-(/root/reference/src/thirdparty/liop/vl_liop.c -> oracle/_ref/libvlliop_ref.so, recipe: oracle/Makefile `ref`),
-so this row of the scope table is PINNED: bit-exact against the compiled reference here, and against the committed
-golden vectors it produced (tests/golden/liop_ref_v1.npz) on machines without the reference tree."""
+(the reference's src/thirdparty/liop/vl_liop.c -> oracle/_ref/libvlliop_ref.so, recipe: oracle/Makefile `ref`),
+so this row of the scope table is PINNED: bit-exact against the golden vectors the compiled reference produced
+(tests/golden/liop_ref_v1.npz, liop_ref_random_v1.npz), and against the compiled reference itself where it is built."""
+import importlib.util
 import os
 
 import numpy as np
-import pytest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+_spec = importlib.util.spec_from_file_location("make_liop_golden", os.path.join(GOLD, "make_liop_golden.py"))
+make_liop_golden = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(make_liop_golden)
 
 
 def test_liop_process_equals_reference_golden(oracle):
@@ -21,19 +24,15 @@ def test_liop_process_equals_reference_golden(oracle):
 
 
 def test_liop_process_equals_compiled_reference(oracle):
-    if not oracle.liop_ref_available():
-        pytest.skip("reference tree absent (GPU box): covered by the golden vectors")
-    rng = np.random.default_rng(11)
-    patches = []
-    for k in range(120):
-        p = rng.random((41, 41)).astype(np.float32)
-        if k % 3 == 1:
-            p = np.floor(p * (2 + k % 7)) / (2 + k % 7)        # exact ties: the order is the quick sort's own
-        if k % 3 == 2:
-            p = np.cumsum(p, 1) / 41
-        patches.append(p.astype(np.float32))
-    patches = np.stack(patches)
-    ref = oracle.liop_ref_process(patches)
+    """Seeded random patches (exact ties among them: the order is the quick sort's own) against the descriptors the
+    compiled reference computed for them, stored in liop_ref_random_v1.npz; where oracle/_ref is built, the reference
+    is run again and must still give the stored descriptors."""
+    g = np.load(os.path.join(GOLD, "liop_ref_random_v1.npz"))
+    patches = make_liop_golden.random_patches()
+    assert make_liop_golden.patches_sha256(patches) == str(g["patches_sha256"]), "the seeded patches changed"
+    ref = g["desc"]
+    if oracle.liop_ref_available():
+        assert np.array_equal(oracle.liop_ref_process(patches).view(np.uint32), ref.view(np.uint32))
     for k in range(len(patches)):
         assert np.array_equal(oracle.liop_process(patches[k]).view(np.uint32), ref[k].view(np.uint32)), "patch %d" % k
     assert np.allclose(np.linalg.norm(ref, axis=1), 1.0, atol=1e-6)
