@@ -215,6 +215,38 @@ int r3d_filter_pairs(r3d_ctx* ctx, int model, double precision_px, uint32_t max_
                      const r3d_matches* putative, const r3d_view_info* views, uint32_t n_views,
                      r3d_matches** out);
 
+/* ---- relative poses (SURVEY.md App. A.9) ----------------------------------------------------------------------- */
+/* openMVG::sfm::RelativePose_Info of one pair, plus what AutomaticInitialPairChoice scores it by. */
+typedef struct {
+  uint32_t I, J; int valid;            /* valid = robustRelativePose returned true */
+  uint32_t n_inliers, n_front;         /* AC-RANSAC inliers; those in front of both cameras (chosen candidate) */
+  double min_nfa, found_residual_precision;  /* ACRANSAC's minNFA (+inf when it never ran); sqrt(errorMax) in pixels (+inf unless it succeeded) */
+  double essential[9], rotation[9], translation[3], center[3];  /* row-major; X_J = R X_I + t, C = -R^T t, |t| = 1 */
+  double median_angle_deg;             /* the (n_front / 2)-th smallest triangulation angle of the front inliers */
+} r3d_relative_pose;
+/* Replaces openMVG::sfm::robustRelativePose(intrinsics_I, intrinsics_J, x_I, x_J, relativePose_info, size_I, size_J,
+ * max_iter) run on every pair of a matches map -- the per-pair step of GlobalSfMReconstructionEngine_RelativeMotions
+ * (Compute_Relative_Rotations), of SfMSceneInitializerStellar and of SequentialSfMReconstructionEngine's
+ * AutomaticInitialPairChoice (src/threads/R3DTriangulationThread.cpp:222-250, :416-441, :492-512):
+ *   ACRANSAC(ACKernelAdaptorEssential<FivePointSolver, EpipolarDistanceError>) with initial_residual_tolerance =
+ *   Square(precision_px) (+inf: the unbounded a-contrario mode, robustRelativePose's default) and max_iter iterations
+ *   (4096 by default) -- exactly r3d_filter_pairs(R3D_MODEL_E, precision_px, max_iter); the pair fails on minNFA >= 0
+ *   or fewer than 2.5 * 5 inliers;
+ *   then estimate_Rt_fromE: the four (R, t) of MotionFromEssential, TriangulateDLT of every inlier's bearing vectors
+ *   under each, the candidate with the most points in front of both cameras (the first maximum; none: the pair fails).
+ * median_angle_deg: the ray angle of AutomaticInitialPairChoice over the n_front inliers, the n_front/2-th smallest
+ * (0-based); the thresholds that decide an initial pair are the caller's.  Bearings come from views[] (pinhole K, no
+ * undistortion, as the E filter); focal <= 0 on either view or <= 5 matches: invalid.  out: num_pairs entries in map
+ * order; essential (K2^T F K1 of the scored F = K2^-T E K1^-1, i.e. the winning 5-point E up to rounding),
+ * n_inliers and found_residual_precision are set whenever AC-RANSAC succeeded.  inliers (may be NULL): the AC-RANSAC inlier map,
+ * identical to r3d_filter_pairs(R3D_MODEL_E) with the same parameters.  The pairs shard over the context's devices
+ * like r3d_filter_pairs; r3d_get_filter_timing then reports the AC-RANSAC kernels as ms_score and the pose kernel
+ * inside ms_device_total.  The host-round AC-RANSAC (R3D_FILTER_HOST_ROUNDS set, or the device sample stream failing
+ * its self-test, r3d_debug_rng_selftest() == 0) does not support this entry: R3D_ERR_UNSUPPORTED. */
+int r3d_relative_poses(r3d_ctx* ctx, const r3d_matches* matches, const r3d_view_info* views, uint32_t n_views,
+                       double precision_px, uint32_t max_iter, r3d_relative_pose* out /* num_pairs entries, map order */,
+                       r3d_matches** inliers /* or NULL */);
+
 /* ---- bundle adjustment --------------------------------------------------------------------- */
 /* Replaces openMVG::sfm::Bundle_Adjustment_Ceres::Adjust as driven by the SfM engines' Process()
  * (src/threads/R3DTriangulationThread.cpp:441, :512, :250).  Default camera model: pinhole radial-K3 (chosen at :398,

@@ -24,7 +24,7 @@ NVCC_FLAGS = [
 ]
 # translation units whose floating-point decisions must match the CPU restatement bit for bit are
 # compiled without FMA contraction
-NO_FMAD = {"acransac_kernels.cu", "acransac_fused.cu", "liop.cu"}
+NO_FMAD = {"acransac_kernels.cu", "acransac_fused.cu", "liop.cu", "relpose.cu"}
 
 
 def sources():

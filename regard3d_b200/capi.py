@@ -4,6 +4,7 @@ Fails loudly: importing works anywhere (the CPU-only tests check the exported sy
 `Context()` raises R3DError when no sm_100 device is present -- there is no CPU fallback.
 """
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -34,6 +35,7 @@ EXPORTS = [
     "r3d_sfm_add_landmark", "r3d_sfm_get_landmark", "r3d_debug_ba_jacobian_model", "r3d_debug_ba_prior", "r3d_sfm_ba_default_options", "r3d_sfm_bundle_adjust",
     "r3d_tracks_build", "r3d_tracks_count", "r3d_tracks_get", "r3d_tracks_in_images", "r3d_tracks_free",
     "r3d_sfm_structure_from_tracks", "r3d_sfm_remove_outliers", "r3d_cascade_prepare", "r3d_debug_cascade_view",
+    "r3d_relative_poses",
 ]
 
 
@@ -75,6 +77,24 @@ def make_views(widths, heights, Ks=None):
         else:
             views[k].focal, views[k].ppx, views[k].ppy = float(Ks[k][0]), float(Ks[k][1]), float(Ks[k][2])
     return views
+
+
+class RelativePose(C.Structure):
+    """r3d_relative_pose (openMVG RelativePose_Info + the initial-pair score)."""
+    _fields_ = [("I", C.c_uint32), ("J", C.c_uint32), ("valid", C.c_int), ("n_inliers", C.c_uint32), ("n_front", C.c_uint32),
+                ("min_nfa", C.c_double), ("found_residual_precision", C.c_double), ("essential", C.c_double * 9),
+                ("rotation", C.c_double * 9), ("translation", C.c_double * 3), ("center", C.c_double * 3),
+                ("median_angle_deg", C.c_double)]
+
+
+# the same layout as a numpy record (what Context.relative_poses returns)
+relative_pose_dtype = np.dtype({
+    "names": [f for f, _ in RelativePose._fields_],
+    "formats": [np.uint32, np.uint32, np.int32, np.uint32, np.uint32, np.float64, np.float64, (np.float64, (3, 3)),
+                (np.float64, (3, 3)), (np.float64, 3), (np.float64, 3), np.float64],
+    "offsets": [getattr(RelativePose, f).offset for f, _ in RelativePose._fields_],
+    "itemsize": C.sizeof(RelativePose),
+})
 
 
 class BAProblem(C.Structure):
@@ -611,6 +631,17 @@ class Context:
         self._check(lib().r3d_filter_pairs(self._h, C.c_int(model), C.c_double(precision_px), C.c_uint32(max_iter),
                                            putative.handle, views, C.c_uint32(n), C.byref(h)))
         return Matches(h)
+
+    def relative_poses(self, matches, widths, heights, Ks, precision_px=math.inf, max_iter=4096, want_inliers=True):
+        """robustRelativePose on every pair of `matches` (Ks: n_views x 3 = focal, ppx, ppy; focal <= 0 = no pinhole
+        intrinsic).  Returns (structured array of relative_pose_dtype in map order, the AC-RANSAC inlier Matches or
+        None)."""
+        views = make_views(widths, heights, Ks)
+        out = np.zeros(matches.num_pairs, relative_pose_dtype)
+        h = C.c_void_p()
+        self._check(lib().r3d_relative_poses(self._h, matches.handle, views, C.c_uint32(len(widths)), C.c_double(precision_px),
+                                             C.c_uint32(max_iter), _p(out), C.byref(h) if want_inliers else None))
+        return out, (Matches(h) if want_inliers else None)
 
     def match_timing(self):
         t = MatchTiming()

@@ -57,13 +57,29 @@ struct AcFusedOut {      // per pair, written by the persistent kernel (acransac
 };
 
 // persistent one-CTA-per-pair ACRANSAC (acransac_fused.cu); `order`: pair ids of one size class, largest first;
-// huge: sort buffers / pool in global scratch (cap entries per CTA of the grid)
+// huge: sort buffers / pool in global scratch (cap entries per CTA of the grid); out_F (essential model only, may be
+// nullptr): 9 doubles per pair, the winning model as scored (F = K2^-T E K1^-1), zeros when no model was ever kept
 size_t acransac_fused_smem_bytes(int model, uint32_t cap, bool huge);
 int acransac_fused_ctas_per_sm(int model, uint32_t cap, bool huge);
 int launch_acransac_fused(r3d_ctx* ctx, DeviceWorker& w, int model, bool huge, const AcPair* pairs, const uint32_t* order,
                           uint32_t n_order, uint32_t* work_counter, const double2* x1, const double2* x2, const float* logc_n,
                           const float* logc_k, uint32_t cap, uint32_t max_iter, double* g_se, uint32_t* g_si, uint32_t* g_pool,
-                          const uint2* matches, uint2* out_matches, AcFusedOut* out, uint32_t grid);
+                          const uint2* matches, uint2* out_matches, AcFusedOut* out, double* out_F, uint32_t grid);
+
+struct RelposeDev {      // per pair, written by k_relpose (relpose.cu)
+  double E[9];           // K2^T F K1 of the winning F (zeros when AC-RANSAC failed)
+  double R[9], t[3], C[3];  // chosen candidate of MotionFromEssential: X_J = R X_I + t, C = -R^T t
+  double median_angle_deg;
+  uint32_t n_front;      // inliers in front of both cameras under the chosen candidate (0: the pair fails)
+  uint32_t pad_;
+};
+
+// relative pose of every pair from its AC-RANSAC result (relpose.cu, k_relpose: one CTA per pair), on the filter's
+// stream: pairs / ac / F (9 doubles per pair) / inlier (i, j) lists as the fused kernel left them; keys / mask:
+// pt_total entries of scratch
+int launch_relpose(r3d_ctx* ctx, DeviceWorker& w, const AcPair* pairs, const AcPointSrc* src, uint32_t n_pairs,
+                   const AcFusedOut* ac, const double* F, const uint2* inl, unsigned long long* keys, uint8_t* mask,
+                   RelposeDev* out);
 
 // x1/x2[pt_ofs + k] = normalised positions of putative match k of every pair (double, like MatchesPairToMat)
 int launch_ac_points(r3d_ctx* ctx, DeviceWorker& w, const AcPair* pairs, const AcPointSrc* src, uint32_t n_pairs,

@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(kFThreads, MODEL == 2 ? 1 : 2) k_acransac_fuse
     const double2* __restrict__ x1, const double2* __restrict__ x2, const float* __restrict__ logc_n,
     const float* __restrict__ logc_k, uint32_t cap, uint32_t max_iter, double* __restrict__ g_se, uint32_t* __restrict__ g_si,
     uint32_t* __restrict__ g_pool, const uint2* __restrict__ matches, uint2* __restrict__ out_matches,
-    AcFusedOut* __restrict__ out) {
+    AcFusedOut* __restrict__ out, double* __restrict__ out_F) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr uint32_t NS = ac_min_samples(MODEL), MAXM = ac_max_models(MODEL);
   typedef typename std::conditional<HUGE, uint32_t, uint16_t>::type PoolT;
@@ -513,6 +513,11 @@ __global__ void __launch_bounds__(kFThreads, MODEL == 2 ? 1 : 2) k_acransac_fuse
       n_out = best_k < c ? best_k : c;
       for (uint32_t i = tid; i < n_out; i += kFThreads) out_matches[pr.pt_ofs + i] = matches[pr.pt_ofs + si[i]];
     }
+    // the winning model (relative poses; nullptr for the filter): F = K2^-T E K1^-1 of the best 5-point E, zeros
+    // when no model was kept
+    if constexpr (MODEL == 2) {
+      if (out_F != nullptr && tid < 9) out_F[(size_t)pair_id * 9 + tid] = have_inliers ? S.bestF[tid] : 0.0;
+    }
     if (tid == 0) {
       AcFusedOut o;
       o.minNFA = minNFA;
@@ -532,11 +537,11 @@ template <int MODEL, bool HUGE>
 static int launch_fused_t(r3d_ctx* ctx, DeviceWorker& w, const AcPair* pairs, const uint32_t* order, uint32_t n_order,
                           uint32_t* work_counter, const double2* x1, const double2* x2, const float* logc_n, const float* logc_k,
                           uint32_t cap, uint32_t max_iter, double* g_se, uint32_t* g_si, uint32_t* g_pool, const uint2* matches,
-                          uint2* out_matches, AcFusedOut* out, uint32_t grid) {
+                          uint2* out_matches, AcFusedOut* out, double* out_F, uint32_t grid) {
   const size_t smem = acransac_fused_smem_bytes(MODEL, cap, HUGE);
   R3D_CUDA_TRY(ctx, cudaFuncSetAttribute(k_acransac_fused<MODEL, HUGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_acransac_fused<MODEL, HUGE><<<grid, kFThreads, smem, w.stream>>>(pairs, order, n_order, work_counter, x1, x2, logc_n, logc_k,
-                                                                      cap, max_iter, g_se, g_si, g_pool, matches, out_matches, out);
+                                                                      cap, max_iter, g_se, g_si, g_pool, matches, out_matches, out, out_F);
   R3D_CUDA_TRY(ctx, cudaGetLastError());
   return R3D_OK;
 }
@@ -553,12 +558,13 @@ int acransac_fused_ctas_per_sm(int model, uint32_t cap, bool huge) {
 int launch_acransac_fused(r3d_ctx* ctx, DeviceWorker& w, int model, bool huge, const AcPair* pairs, const uint32_t* order,
                           uint32_t n_order, uint32_t* work_counter, const double2* x1, const double2* x2, const float* logc_n,
                           const float* logc_k, uint32_t cap, uint32_t max_iter, double* g_se, uint32_t* g_si, uint32_t* g_pool,
-                          const uint2* matches, uint2* out_matches, AcFusedOut* out, uint32_t grid) {
+                          const uint2* matches, uint2* out_matches, AcFusedOut* out, double* out_F, uint32_t grid) {
   if (!n_order) return R3D_OK;
+  if (out_F != nullptr && model != 2) return fail(ctx, R3D_ERR_INVALID, "launch_acransac_fused: the winning-model output needs the E model");
 #define R3D_FUSED_CASE(MD, HG)                                                                                          \
   if (model == MD && huge == HG)                                                                                        \
     return launch_fused_t<MD, HG>(ctx, w, pairs, order, n_order, work_counter, x1, x2, logc_n, logc_k, cap, max_iter, \
-                                  g_se, g_si, g_pool, matches, out_matches, out, grid);
+                                  g_se, g_si, g_pool, matches, out_matches, out, out_F, grid);
   R3D_FUSED_CASE(0, false) R3D_FUSED_CASE(0, true) R3D_FUSED_CASE(1, false) R3D_FUSED_CASE(1, true)
   R3D_FUSED_CASE(2, false) R3D_FUSED_CASE(2, true)
 #undef R3D_FUSED_CASE

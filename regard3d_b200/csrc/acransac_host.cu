@@ -107,13 +107,25 @@ std::vector<uint32_t> st_src(const std::vector<PairState>& st) {
   return v;
 }
 
+}  // namespace
+
+// Relative poses (r3d_relative_poses): what the essential AC-RANSAC leaves on the device feeds k_relpose on the same
+// stream, before the one synchronisation; the per-pair results land in out[] (indexed by pair of the putative map)
+struct RelposeIo {
+  const AcPointSrc* d_src = nullptr;  // positions and intrinsics of each pair's views (set by filter_pairs_model)
+  r3d_relative_pose* out = nullptr;
+};
+
+namespace {
+
 // The device-resident ACRANSAC (acransac_fused.cu): the pairs are cut into size classes (shared-memory sort capacity
 // 1024 ... 16384 putative matches; beyond that the "huge" class sorts in global scratch), one persistent launch per
 // class, largest pairs first; ONE synchronisation, then the inlier lists come back through pinned staging.
+// rp != nullptr (essential model): the relative-pose kernel runs after the AC-RANSAC launches.
 int run_fused(r3d_ctx* ctx, DeviceWorker& w, int model, uint32_t max_iter, const r3d_matches* put, const std::vector<uint32_t>& src,
               const std::vector<AcPair>& hpairs, const AcPair* d_pairs, const double2* d_x1, const double2* d_x2,
               const uint2* d_match, const float* d_logc_n, const float* d_logc_k, uint32_t pt_total, uint32_t sizeSample,
-              double t_begin, r3d_filter_timing& T, std::vector<std::vector<r3d_indmatch>>& result) {
+              double t_begin, r3d_filter_timing& T, std::vector<std::vector<r3d_indmatch>>& result, RelposeIo* rp) {
   const uint32_t n = (uint32_t)hpairs.size();
   constexpr int kClasses = 6;  // caps 1024, 2048, 4096, 8192, 16384, huge
   std::vector<uint32_t> order[kClasses];
@@ -141,11 +153,21 @@ int run_fused(r3d_ctx* ctx, DeviceWorker& w, int model, uint32_t max_iter, const
   R3D_CUDA_TRY(ctx, d_work.ensure(kClasses));
   R3D_CUDA_TRY(ctx, d_out.ensure(n));
   R3D_CUDA_TRY(ctx, d_outm.ensure(pt_total));
+  DevBuf<double> d_F(w);
+  DevBuf<RelposeDev> d_rp(w);
+  DevBuf<unsigned long long> d_keys(w);
+  DevBuf<uint8_t> d_mask(w);
+  if (rp) {
+    R3D_CUDA_TRY(ctx, d_F.ensure((size_t)n * 9));
+    R3D_CUDA_TRY(ctx, d_rp.ensure(n));
+    R3D_CUDA_TRY(ctx, d_keys.ensure(pt_total));
+    R3D_CUDA_TRY(ctx, d_mask.ensure(pt_total));
+  }
   R3D_CUDA_TRY(ctx, cudaMemcpyAsync(d_order.p, horder.data(), horder.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, w.stream));
   R3D_CUDA_TRY(ctx, cudaMemsetAsync(d_work.p, 0, kClasses * sizeof(uint32_t), w.stream));
-  cudaEvent_t ev[2];
+  cudaEvent_t ev[3];
   for (auto& e : ev) R3D_CUDA_TRY(ctx, cudaEventCreate(&e));
-  struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 2; ++i) cudaEventDestroy(e[i]); } } evg{ev};
+  struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } evg{ev};
   R3D_CUDA_TRY(ctx, cudaEventRecord(ev[0], w.stream));
   // launch geometry of every class first: the scratch buffers are shared by the launches (same stream) and must not move
   uint32_t caps[kClasses] = {0}, grids[kClasses] = {0};
@@ -175,17 +197,47 @@ int run_fused(r3d_ctx* ctx, DeviceWorker& w, int model, uint32_t max_iter, const
     const uint32_t cnt = class_ofs[c + 1] - class_ofs[c];
     if (!cnt) continue;
     int rc = launch_acransac_fused(ctx, w, model, c == 5, d_pairs, d_order.p + class_ofs[c], cnt, d_work.p + c, d_x1, d_x2, d_logc_n,
-                                   d_logc_k, caps[c], max_iter, d_se.p, d_si.p, d_pool.p, d_match, d_outm.p, d_out.p, grids[c]);
+                                   d_logc_k, caps[c], max_iter, d_se.p, d_si.p, d_pool.p, d_match, d_outm.p, d_out.p,
+                                   rp ? d_F.p : nullptr, grids[c]);
     if (rc) return rc;
     T.kernel_launches += 1;
   }
   R3D_CUDA_TRY(ctx, cudaEventRecord(ev[1], w.stream));
+  std::vector<RelposeDev> hrp;
+  if (rp) {
+    int rc = launch_relpose(ctx, w, d_pairs, rp->d_src, n, d_out.p, d_F.p, d_outm.p, d_keys.p, d_mask.p, d_rp.p);
+    if (rc) return rc;
+    T.kernel_launches += 1;
+    R3D_CUDA_TRY(ctx, cudaEventRecord(ev[2], w.stream));
+    hrp.resize(n);
+    R3D_CUDA_TRY(ctx, cudaMemcpyAsync(hrp.data(), d_rp.p, (size_t)n * sizeof(RelposeDev), cudaMemcpyDeviceToHost, w.stream));
+  }
   std::vector<AcFusedOut> hout(n);
   R3D_CUDA_TRY(ctx, cudaMemcpyAsync(hout.data(), d_out.p, (size_t)n * sizeof(AcFusedOut), cudaMemcpyDeviceToHost, w.stream));
   R3D_CUDA_TRY(ctx, cudaStreamSynchronize(w.stream));
-  float ms = 0.f;
+  float ms = 0.f, ms_total = 0.f;
   cudaEventElapsedTime(&ms, ev[0], ev[1]);
   T.ms_score = ms;
+  if (rp) {
+    cudaEventElapsedTime(&ms_total, ev[0], ev[2]);
+    for (uint32_t a = 0; a < n; ++a) {  // RelativePose_Info of every pair that ran
+      const AcFusedOut& o = hout[a];
+      const RelposeDev& d = hrp[a];
+      r3d_relative_pose& r = rp->out[src[a]];
+      r.min_nfa = o.minNFA;
+      if (!(o.minNFA < 0) || !((double)o.n_inliers > sizeSample * 2.5)) continue;
+      r.found_residual_precision = std::sqrt(o.errorMax);
+      r.n_inliers = o.n_inliers;
+      std::memcpy(r.essential, d.E, sizeof(r.essential));
+      if (d.n_front == 0) continue;  // no candidate puts a point in front of both cameras
+      r.valid = 1;
+      r.n_front = d.n_front;
+      std::memcpy(r.rotation, d.R, sizeof(r.rotation));
+      std::memcpy(r.translation, d.t, sizeof(r.translation));
+      std::memcpy(r.center, d.C, sizeof(r.center));
+      r.median_angle_deg = d.median_angle_deg;
+    }
+  }
   T.ms_solve = 0.0;
   T.rounds = 1;
   for (const AcFusedOut& o : hout) T.hypotheses += o.iterations;
@@ -258,7 +310,7 @@ int run_fused(r3d_ctx* ctx, DeviceWorker& w, int model, uint32_t max_iter, const
   (void)put;
   if (getenv("R3D_DEBUG_TIMING"))
     fprintf(stderr, "[r3d] fused filter total %.2f ms (kernel %.2f, results back %.2f)\n", now_ms() - t_begin, T.ms_score, now_ms() - t_after_kernel);
-  T.ms_device_total = T.ms_score;
+  T.ms_device_total = rp ? (double)ms_total : T.ms_score;
   T.ms_host = now_ms() - t_begin - T.ms_device_total;
   return R3D_OK;
 }
@@ -268,7 +320,7 @@ int run_fused(r3d_ctx* ctx, DeviceWorker& w, int model, uint32_t max_iter, const
 // pairs [p0, p1) of the putative map on worker w; result (sized by the caller to the whole map) is indexed by pair
 int filter_pairs_model(r3d_ctx* ctx, DeviceWorker& w, int model, double precision_px, uint32_t max_iter, const r3d_matches* put,
                    const r3d_view_info* views, uint32_t n_views, uint64_t p0, uint64_t p1, r3d_filter_timing& T,
-                   std::vector<std::vector<r3d_indmatch>>& result) {
+                   std::vector<std::vector<r3d_indmatch>>& result, RelposeIo* rp = nullptr) {
   R3D_CUDA_TRY(ctx, cudaSetDevice(w.device));
   T = r3d_filter_timing{};
   const double t_begin = now_ms();
@@ -311,6 +363,9 @@ int filter_pairs_model(r3d_ctx* ctx, DeviceWorker& w, int model, double precisio
   // the persistent per-pair kernel draws the sample stream on the device; it needs the restated
   // std::uniform_int_distribution to agree with this process's <random> (acransac_rng.cuh)
   const bool use_fused = rng_selftest() && !getenv("R3D_FILTER_HOST_ROUNDS");
+  if (rp && !use_fused)
+    return fail(ctx, R3D_ERR_UNSUPPORTED, "r3d_relative_poses: needs the device-resident AC-RANSAC (R3D_FILTER_HOST_ROUNDS is set "
+                                          "or the device sample stream failed its self-test)");
   // log-combinatorial tables (float, upstream makelogcombi_n / makelogcombi_k).  logcombi(k,n) is a
   // running float sum over i = 1..min(k,n-k): its partial sums ARE the entries for smaller k, so one
   // O(n) pass reproduces the upstream O(n^2) table bit for bit.
@@ -467,9 +522,11 @@ int filter_pairs_model(r3d_ctx* ctx, DeviceWorker& w, int model, double precisio
   R3D_CUDA_TRY(ctx, cudaMemcpyAsync(d_logc_k.p, hlogc_k.data(), hlogc_k.size() * sizeof(float), cudaMemcpyHostToDevice, w.stream));
 
   if (getenv("R3D_DEBUG_TIMING")) fprintf(stderr, "[r3d] filter host set-up + point upload: %.2f ms\n", now_ms() - t_begin);
-  if (use_fused)
+  if (use_fused) {
+    if (rp) rp->d_src = d_src.p;
     return run_fused(ctx, w, model, max_iter, put, st_src(st), hpairs, d_pairs.p, d_x1.p, d_x2.p, d_match.p, d_logc_n.p, d_logc_k.p,
-                     (uint32_t)n_match_total, sizeSample, t_begin, T, result);
+                     (uint32_t)n_match_total, sizeSample, t_begin, T, result, rp);
+  }
 
   cudaEvent_t ev[3];
   for (auto& e : ev) R3D_CUDA_TRY(ctx, cudaEventCreate(&e));
@@ -656,17 +713,14 @@ using namespace r3d;
 // (acransac_rng.cuh) reproduces this process's <random>, i.e. when the filter runs fully on the device.
 extern "C" int r3d_debug_rng_selftest(void) { return rng_selftest() ? 1 : 0; }
 
-extern "C" int r3d_filter_pairs(r3d_ctx* ctx, int model, double precision_px, uint32_t max_iter, const r3d_matches* putative,
-                                const r3d_view_info* views, uint32_t n_views, r3d_matches** out) {
-  if (!ctx || !putative || !views || !out) return fail(ctx, R3D_ERR_INVALID, "r3d_filter_pairs: bad arguments");
-  *out = nullptr;
-  if (model != R3D_MODEL_F && model != R3D_MODEL_H && model != R3D_MODEL_E)
-    return fail(ctx, R3D_ERR_INVALID, "r3d_filter_pairs: unknown model");
-  const int internal = model == R3D_MODEL_F ? 0 : (model == R3D_MODEL_H ? 1 : 2);
+namespace {
+
+// image pairs are independent: cut the map into contiguous ranges of equal putative-match counts, one per device
+// of the context (every device holds all positions), no collective -- the same rule as r3d_match_pairs.
+// run(worker, p0, p1, timing) filters pairs [p0, p1); the context's filter timing becomes the slowest device's.
+template <typename Run>
+int shard_pairs(r3d_ctx* ctx, const r3d_matches* putative, Run run) {
   const uint64_t P_all = putative->pairs.size() / 2;
-  std::vector<std::vector<r3d_indmatch>> res(P_all);
-  // image pairs are independent: cut the map into contiguous ranges of equal putative-match counts, one per device
-  // of the context (every device holds all positions), no collective -- the same rule as r3d_match_pairs
   const size_t nw = ctx->workers.size();
   std::vector<uint64_t> cut(nw + 1, 0);
   {
@@ -679,37 +733,79 @@ extern "C" int r3d_filter_pairs(r3d_ctx* ctx, int model, double precision_px, ui
   std::vector<int> rcs(nw, R3D_OK);
   std::vector<r3d_filter_timing> tms(nw);
   if (nw == 1) {
-    rcs[0] = filter_pairs_model(ctx, ctx->workers[0], internal, precision_px, max_iter, putative, views, n_views, 0, P_all, tms[0], res);
+    rcs[0] = run(ctx->workers[0], (uint64_t)0, P_all, tms[0]);
   } else {
     std::vector<std::thread> th;
     for (size_t k = 0; k < nw; ++k)
-      th.emplace_back([&, k]() {
-        rcs[k] = filter_pairs_model(ctx, ctx->workers[k], internal, precision_px, max_iter, putative, views, n_views, cut[k], cut[k + 1],
-                                    tms[k], res);
-      });
+      th.emplace_back([&, k]() { rcs[k] = run(ctx->workers[k], cut[k], cut[k + 1], tms[k]); });
     for (auto& t : th) t.join();
   }
   for (int rc : rcs)
     if (rc) return rc;
-  {
-    r3d_filter_timing sum{};
-    for (const r3d_filter_timing& t : tms) {
-      sum.ms_solve = std::max(sum.ms_solve, t.ms_solve);
-      sum.ms_score = std::max(sum.ms_score, t.ms_score);
-      sum.ms_device_total = std::max(sum.ms_device_total, t.ms_device_total);
-      sum.ms_host = std::max(sum.ms_host, t.ms_host);
-      sum.kernel_launches += t.kernel_launches;
-      sum.hypotheses += t.hypotheses;
-      sum.rounds = std::max(sum.rounds, t.rounds);
-    }
-    ctx->filter_timing = sum;
+  r3d_filter_timing sum{};
+  for (const r3d_filter_timing& t : tms) {
+    sum.ms_solve = std::max(sum.ms_solve, t.ms_solve);
+    sum.ms_score = std::max(sum.ms_score, t.ms_score);
+    sum.ms_device_total = std::max(sum.ms_device_total, t.ms_device_total);
+    sum.ms_host = std::max(sum.ms_host, t.ms_host);
+    sum.kernel_launches += t.kernel_launches;
+    sum.hypotheses += t.hypotheses;
+    sum.rounds = std::max(sum.rounds, t.rounds);
   }
+  ctx->filter_timing = sum;
+  return R3D_OK;
+}
+
+// the pairs that kept inliers, in map order (pairs whose estimation failed disappear from the map)
+r3d_matches* inlier_map(const r3d_matches* putative, std::vector<std::vector<r3d_indmatch>>& res) {
   r3d_matches* m = new r3d_matches();
   const uint64_t P = putative->pairs.size() / 2;
   for (uint64_t p = 0; p < P; ++p) {
-    if (res[p].empty()) continue;  // pairs whose estimation failed disappear from the map
+    if (res[p].empty()) continue;
     m->push(putative->pairs[2 * p], putative->pairs[2 * p + 1], std::move(res[p]));
   }
-  *out = m;
+  return m;
+}
+
+}  // namespace
+
+extern "C" int r3d_filter_pairs(r3d_ctx* ctx, int model, double precision_px, uint32_t max_iter, const r3d_matches* putative,
+                                const r3d_view_info* views, uint32_t n_views, r3d_matches** out) {
+  if (!ctx || !putative || !views || !out) return fail(ctx, R3D_ERR_INVALID, "r3d_filter_pairs: bad arguments");
+  *out = nullptr;
+  if (model != R3D_MODEL_F && model != R3D_MODEL_H && model != R3D_MODEL_E)
+    return fail(ctx, R3D_ERR_INVALID, "r3d_filter_pairs: unknown model");
+  const int internal = model == R3D_MODEL_F ? 0 : (model == R3D_MODEL_H ? 1 : 2);
+  std::vector<std::vector<r3d_indmatch>> res(putative->pairs.size() / 2);
+  const int rc = shard_pairs(ctx, putative, [&](DeviceWorker& w, uint64_t p0, uint64_t p1, r3d_filter_timing& T) {
+    return filter_pairs_model(ctx, w, internal, precision_px, max_iter, putative, views, n_views, p0, p1, T, res);
+  });
+  if (rc) return rc;
+  *out = inlier_map(putative, res);
+  return R3D_OK;
+}
+
+extern "C" int r3d_relative_poses(r3d_ctx* ctx, const r3d_matches* matches, const r3d_view_info* views, uint32_t n_views,
+                                  double precision_px, uint32_t max_iter, r3d_relative_pose* out, r3d_matches** inliers) {
+  if (!ctx || !matches || !views || !out) return fail(ctx, R3D_ERR_INVALID, "r3d_relative_poses: bad arguments");
+  if (inliers) *inliers = nullptr;
+  if (!(precision_px > 0.0)) return fail(ctx, R3D_ERR_INVALID, "r3d_relative_poses: precision_px must be > 0 (or +inf)");
+  const uint64_t P = matches->pairs.size() / 2;
+  for (uint64_t p = 0; p < P; ++p) {  // pairs that never reach the estimation keep this: invalid, nothing found
+    r3d_relative_pose& r = out[p];
+    std::memset(&r, 0, sizeof(r));
+    r.I = matches->pairs[2 * p];
+    r.J = matches->pairs[2 * p + 1];
+    r.min_nfa = std::numeric_limits<double>::infinity();
+    r.found_residual_precision = std::numeric_limits<double>::infinity();
+  }
+  std::vector<std::vector<r3d_indmatch>> res(P);
+  const int rc = shard_pairs(ctx, matches, [&](DeviceWorker& w, uint64_t p0, uint64_t p1, r3d_filter_timing& T) {
+    RelposeIo io;
+    io.out = out;
+    return filter_pairs_model(ctx, w, 2, precision_px, max_iter, matches, views, n_views, p0, p1, T, res, &io);
+  });
+  if (rc) return rc;
+  if (inliers) *inliers = inlier_map(matches, res);
   return R3D_OK;
 }
